@@ -23,6 +23,9 @@ Reported on ONE JSON line (see the task contract):
   parity     view 0 against the oracle: pixels over 1e-4, fragile fraction, worst non-fragile / fragile error (N = 1)
 `--impl reference` times that CPU port alone (the reference's rasterizer is an absent external CUDA extension
 and the reference has no CPU path of its own: SURVEY.md section 0, BASELINE.md section 2-3).
+`--dump-outputs DIR` writes what the last timed forward step returned (DIR/color.npy, DIR/radii.npy; suffixed _rank<r>
+under N > 1), at most DUMP_BUDGET bytes over all ranks (see write_outputs).  The inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -125,6 +128,37 @@ def host_threads() -> int:
     return max(1, n)
 
 
+DUMP_BUDGET = 64 * 10**6   # bytes --dump-outputs may write, all ranks together
+
+
+def write_outputs(out_dir, outputs, world=1, rank=0, budget=DUMP_BUDGET):
+    """Writes `outputs` (name -> array) as out_dir/<name>.npy in float32, suffixed _rank<r> under N > 1, in at most
+    budget // world bytes per rank.  Arrays over that share are all replaced by a fixed sample of their elements, seeded
+    by the rank and so the same in every run of the same workload: the values in <name>.npy, their flat indices into the
+    full array in <name>_index.npy (float64, exact below 2**53).  Returns the bytes written."""
+    import numpy as np
+    share = budget // world
+    header = 128                 # .npy header of these arrays
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in outputs.items()}
+    if sum(a.nbytes + header for a in arrays.values()) > share:
+        # one sampling fraction for all arrays: 4 bytes of value + 8 of index per kept element
+        frac = max(0, share - 2 * header * len(arrays)) / (12 * sum(a.size for a in arrays.values()))
+        rng = np.random.default_rng(rank)
+        sampled = {}
+        for k, a in arrays.items():
+            idx = np.unique(rng.integers(0, a.size, int(a.size * frac)))
+            sampled[k], sampled[k + "_index"] = a.reshape(-1)[idx], idx.astype(np.float64)
+        arrays = sampled
+    os.makedirs(out_dir, exist_ok=True)
+    written = 0
+    for k, a in arrays.items():
+        path = os.path.join(out_dir, k + (f"_rank{rank}" if world > 1 else "") + ".npy")
+        np.save(path, a)
+        written += os.path.getsize(path)
+    assert written <= share, f"--dump-outputs wrote {written} bytes, over this rank's {share}"
+    return written
+
+
 def run_reference(args):
     """CPU arm: the oracle port on the host cores, one whole view of the workload per step."""
     import numpy as np
@@ -169,7 +203,11 @@ def main():
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-c4", action="store_true", help="skip the C4 (2M x 32 views x 512x512) strong-scaling block")
     ap.add_argument("--no-moving", action="store_true", help="skip the moving-cloud leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed forward step returned (color, radii) to DIR/<name>.npy, in float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global P_GAUSS, VIEWS, HW, WORKLOAD
     P_GAUSS, VIEWS, HW, WORKLOAD = WORKLOADS[args.workload]
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
@@ -306,14 +344,16 @@ def main():
 
     per_rank_ms = {}
 
-    def timed(fn, steps, warmup, tag=None):
+    def timed(fn, steps, warmup, tag=None, keep_last=False):
+        """Device ms of `steps` calls of fn (max over ranks); with keep_last, also what the last call returned."""
         for _ in range(warmup):
             fn()
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         e1.record(stream)
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -322,7 +362,7 @@ def main():
             dist.all_gather(every, ms)                      # each rank's own device time: what the MAX below is taken over
             per_rank_ms[tag] = [float(t.item()) / steps for t in every]
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return (float(ms.item()), last) if keep_last else float(ms.item())
 
     gauss_per_step = P_GAUSS * VIEWS * world
 
@@ -341,8 +381,10 @@ def main():
 
     sampler = ClockSampler(local)
     sampler.start()
-    ms_fwd = timed(fwd, args.steps, args.warmup, "fwd")
+    ms_fwd, last_fwd = timed(fwd, args.steps, args.warmup, "fwd", keep_last=True)
     launches_fwd = rasterizer.last_stats(dev)["kernel_launches"]   # of the last timed step (steady state)
+    dump = {name: t.float().cpu().numpy() for name, t in zip(("color", "radii"), last_fwd)} if args.dump_outputs else None
+    del last_fwd
     ms_e2e = timed(e2e, args.steps, args.warmup, "e2e")
     launches_e2e = rasterizer.last_stats(dev)["kernel_launches"]   # 4 with the split pipeline (k_sh_colour), else 3
     ms_fb = timed(fwd_bwd, args.steps, args.warmup, "fwd_bwd")
@@ -692,6 +734,8 @@ def main():
         }
         sys.stdout.flush()
         print(json.dumps(line), flush=True)
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump, world, rank)
     if world > 1:
         dist.destroy_process_group()
 

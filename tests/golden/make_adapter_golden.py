@@ -84,6 +84,22 @@ def make_inputs(seed, b, v, h, w, sh_degree, proper=True, srf=1, spp=1):
     return dict(extrinsics=ext, intrinsics=intr, coordinates=coords, depths=depths, opacities=opac, raw_gaussians=raw)
 
 
+def make_weights(seed, shapes):
+    """Weights w_k of the loss sum_k <w_k, out_k> whose gradients the fixture records, for outputs of the given shapes."""
+    g = torch.Generator().manual_seed(100 + seed)
+    return {k: torch.randn(s, generator=g) for k, s in shapes.items()}
+
+
+def sh_rotation_used(extrinsics, b, v, sh_degree):
+    """The block-diagonal Wigner-D matrices the e3nn stub hands the reference's rotate_sh (identity for improper
+    rotations, which rotate_sh leaves alone)."""
+    rot = extrinsics[..., :3, :3].reshape(b, v, 3, 3)
+    d_sh = (sh_degree + 1) ** 2
+    if rotations_are_proper(rot):
+        return sh_rotation_blocks(rot, d_sh)
+    return torch.eye(d_sh).expand(b, v, d_sh, d_sh)
+
+
 CASES = {
     # name: (seed, b, v, h, w, sh_degree, proper rotations)
     "adapter_pf3plat": (0, 1, 2, 6, 8, 4, True),       # PF3plat: sh_degree 4, two context views
@@ -100,18 +116,12 @@ def main():
         adapter = ref.GaussianAdapter(ref.GaussianAdapterCfg(gaussian_scale_min=0.5, gaussian_scale_max=15.0, sh_degree=deg))
         out = adapter.forward(leaves["extrinsics"], leaves["intrinsics"], leaves["coordinates"], leaves["depths"],
                               leaves["opacities"], leaves["raw_gaussians"], (h, w))
-        g = torch.Generator().manual_seed(100 + seed)
         outs = dict(means=out.means, covariances=out.covariances, harmonics=out.harmonics, scales=out.scales,
                     rotations=out.rotations)
-        weights = {k: torch.randn(t.shape, generator=g) for k, t in outs.items()}
+        weights = make_weights(seed, {k: t.shape for k, t in outs.items()})
         loss = sum((weights[k] * outs[k]).sum() for k in outs)
         loss.backward()
-        rot = inp["extrinsics"][..., :3, :3].reshape(b, v, 3, 3)
-        d_sh = (deg + 1) ** 2
-        if rotations_are_proper(rot):
-            dmat = sh_rotation_blocks(rot, d_sh)
-        else:
-            dmat = torch.eye(d_sh).expand(b, v, d_sh, d_sh)
+        dmat = sh_rotation_used(inp["extrinsics"], b, v, deg)
         arrays = {f"in_{k}": t.numpy() for k, t in inp.items()}
         arrays.update({f"out_{k}": t.detach().numpy() for k, t in outs.items()})
         arrays.update({f"w_{k}": t.numpy() for k, t in weights.items()})

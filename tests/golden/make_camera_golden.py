@@ -3,8 +3,11 @@
 RECORDING stand-in for `diff_gaussian_rasterization`: the stub rasterizer stores the GaussianRasterizationSettings it is
 handed for every view (viewmatrix, projmatrix, campos, tanfovx, tanfovy -- everything lines 64-112 compute) and returns
 blank images.  The fixture therefore pins pf3plat_b200.cameras.make_view_batch / gs_view_batch to the reference's own glue.
+Also writes tests/golden/operator_calls.npz: the raw arguments of every operator call of the three call sites
+(record_operator_calls).
 Only runs in the build container (needs /root/reference).   Usage: python tests/golden/make_camera_golden.py"""
 import importlib.util
+import json
 import os
 import sys
 import types
@@ -95,9 +98,8 @@ def load_reference_decoder():
 DECODER_KEYS = ("viewmatrix", "projmatrix", "campos", "tanfov", "means", "cov6", "bg", "opacities", "colors", "shs", "ints")
 
 
-def run_reference_decoder(b=2, v=3, G=2, depth_mode="depth"):
-    """Inputs and the recorded operator calls of one DecoderSplattingCUDA.forward (colour pass, then depth pass)."""
-    dec_mod, types_mod = load_reference_decoder()
+def decoder_inputs(b=2, v=3, G=2):
+    """The inputs run_reference_decoder hands DecoderSplattingCUDA.forward: b scenes of G Gaussians, v views each."""
     ext, intr, near, far = make_cameras(21, b * v)
     g = torch.Generator().manual_seed(22)
     means = torch.randn(b, G, 3, generator=g).abs() + 0.5
@@ -105,15 +107,23 @@ def run_reference_decoder(b=2, v=3, G=2, depth_mode="depth"):
     cov = a @ a.transpose(-1, -2)
     sh = torch.randn(b, G, 3, 25, generator=g)
     opac = torch.rand(b, G, generator=g)
+    r4 = lambda t: t.reshape(b, v, *t.shape[1:])
+    return dict(extrinsics=r4(ext), intrinsics=r4(intr), near=r4(near), far=r4(far), means=means, covariances=cov, sh=sh,
+                opacities=opac)
+
+
+def run_reference_decoder(b=2, v=3, G=2, depth_mode="depth"):
+    """Inputs and the recorded operator calls of one DecoderSplattingCUDA.forward (colour pass, then depth pass)."""
+    dec_mod, types_mod = load_reference_decoder()
+    inputs = decoder_inputs(b, v, G)
     cfg = types.SimpleNamespace(background_color=[0.1, 0.2, 0.3])
     dec = dec_mod.DecoderSplattingCUDA(dec_mod.DecoderSplattingCUDACfg(name="splatting_cuda"), cfg)
     RECORDED.clear()
-    r4 = lambda t: t.reshape(b, v, *t.shape[1:])
-    dec.forward(types_mod.Gaussians(means, cov, sh, opac), r4(ext), r4(intr), r4(near), r4(far), (16, 24), depth_mode=depth_mode)
+    i = inputs
+    dec.forward(types_mod.Gaussians(i["means"], i["covariances"], i["sh"], i["opacities"]), i["extrinsics"],
+                i["intrinsics"], i["near"], i["far"], (16, 24), depth_mode=depth_mode)
     rec = {k: [r[k] for r in RECORDED] for k in DECODER_KEYS}
     RECORDED.clear()
-    inputs = dict(extrinsics=r4(ext), intrinsics=r4(intr), near=r4(near), far=r4(far), means=means, covariances=cov, sh=sh,
-                  opacities=opac)
     return inputs, rec
 
 
@@ -138,9 +148,9 @@ def make_cameras(seed, B):
     return ext, intr, near, far
 
 
-def main():
-    mod = load_reference_render_cuda()
-    B, G = 9, 2
+def glue_inputs(B=9, G=2):
+    """The cameras and Gaussians of main(): render_cuda gets them as they are, render_depth_cuda the same cameras with
+    means.abs() + 0.5, render_cuda_orthographic only the first scene's Gaussians (with the camera of ortho_inputs())."""
     ext, intr, near, far = make_cameras(12, B)
     g = torch.Generator().manual_seed(13)
     means = torch.randn(B, G, 3, generator=g)
@@ -148,6 +158,75 @@ def main():
     cov = a @ a.transpose(-1, -2)
     sh = torch.randn(B, G, 3, 25, generator=g)
     opac = torch.rand(B, G, generator=g)
+    return ext, intr, near, far, means, cov, sh, opac
+
+
+class _RawSettings(dict):
+    """Stand-in for GaussianRasterizationSettings that keeps the keyword arguments exactly as they were passed."""
+
+    def __init__(self, **kwargs):
+        super().__init__(kwargs)
+
+
+class _RawRecorder:
+    """Stand-in for GaussianRasterizer that keeps its settings and the keyword arguments of every call as handed over."""
+
+    def __init__(self, raster_settings):
+        self.s = raster_settings
+
+    def __call__(self, **kwargs):
+        OPERATOR_CALLS.append((dict(self.s), kwargs))
+        return (torch.zeros(3, self.s["image_height"], self.s["image_width"]),
+                torch.zeros(kwargs["means3D"].shape[0], dtype=torch.int32))
+
+
+OPERATOR_CALLS: list = []
+
+
+def record_operator_calls():
+    """Every operator call of the reference's three call sites (render_cuda, render_cuda_orthographic, and render_cuda
+    again through render_depth_cuda) on a small synthetic scene, argument by argument: tensors as arrays (with
+    requires_grad), Python scalars with their type.  tests/test_capi_cpu.py replays them against this repository's
+    `diff_gaussian_rasterization`."""
+    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+    from pf3plat_b200.synthetic import make_scene
+    mod = load_reference_render_cuda()
+    mod.GaussianRasterizationSettings, mod.GaussianRasterizer = _RawSettings, _RawRecorder
+    sc = make_scene(64, 2, 32, 32)
+    rep = lambda t: t[None].expand(2, *t.shape)
+    one = lambda t: t[:1]
+    OPERATOR_CALLS.clear()
+    mod.render_cuda(sc.extrinsics, sc.intrinsics, sc.near, sc.far, sc.image_shape, sc.background, rep(sc.means),
+                    rep(sc.covariances), rep(sc.harmonics), rep(sc.opacities))
+    mod.render_depth_cuda(sc.extrinsics, sc.intrinsics, sc.near, sc.far, sc.image_shape, rep(sc.means),
+                          rep(sc.covariances), rep(sc.opacities), mode="disparity")
+    mod.render_cuda_orthographic(one(sc.extrinsics), torch.tensor([2.0]), torch.tensor([2.0]), one(sc.near), one(sc.far),
+                                 sc.image_shape, one(sc.background), one(rep(sc.means)), one(rep(sc.covariances)),
+                                 one(rep(sc.harmonics)), one(rep(sc.opacities)))
+    arrays, kinds = {}, {}
+    for i, (settings, call) in enumerate(OPERATOR_CALLS):
+        for part, args in (("settings", settings), ("call", call)):
+            for name, v in args.items():
+                key = f"c{i}.{part}.{name}"
+                if isinstance(v, torch.Tensor):
+                    arrays[key] = v.detach().numpy()
+                    kinds[key] = "tensor_grad" if v.requires_grad else "tensor"
+                elif v is None:
+                    kinds[key] = "none"
+                else:
+                    arrays[key] = np.array(v)
+                    kinds[key] = type(v).__name__
+    arrays["kinds"] = np.array(json.dumps(kinds))
+    OPERATOR_CALLS.clear()
+    path = os.path.join(HERE, "operator_calls.npz")
+    np.savez_compressed(path, **arrays)
+    print(len(kinds), "arguments", os.path.getsize(path), "bytes")
+
+
+def main():
+    mod = load_reference_render_cuda()
+    B = 9
+    ext, intr, near, far, means, cov, sh, opac = glue_inputs(B)
     arrays = dict(extrinsics=ext.numpy(), intrinsics=intr.numpy(), near=near.numpy(), far=far.numpy(),
                   means=means.numpy(), covariances=cov.numpy())
     for tag, si in (("si", True), ("raw", False)):
@@ -192,6 +271,7 @@ def main():
     path = os.path.join(HERE, "camera_glue.npz")
     np.savez_compressed(path, **arrays)
     print({k: v.shape for k, v in arrays.items()}, os.path.getsize(path), "bytes")
+    record_operator_calls()
 
 
 if __name__ == "__main__":

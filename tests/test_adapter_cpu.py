@@ -1,6 +1,6 @@
 """Pins the adapter oracle (oracle/adapter_oracle.py) to the REFERENCE's own outputs: the golden fixtures were
-produced by /root/reference/src/model/encoder/common/gaussian_adapter.py itself (tests/golden/make_adapter_golden.py).
-Also: the SH-rotation helper's algebra, and -- in the build container only -- a live re-run of the reference module."""
+produced by the reference's src/model/encoder/common/gaussian_adapter.py itself (tests/golden/make_adapter_golden.py).
+Also: the SH-rotation helper's algebra, and that the generating script still feeds the reference what the fixtures hold."""
 import os
 import sys
 
@@ -70,25 +70,23 @@ def test_wigner_matrices_are_orthogonal_homomorphic_and_equal_the_rotation_for_d
     assert (sh_rotation.rotate_sh(sh, rot * 1.1) - sh).abs().max() < 1e-13
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/model/encoder/common/gaussian_adapter.py"),
-                    reason="reference tree only exists in the build container")
 def test_fixtures_are_what_the_reference_module_produces_today():
-    """Re-runs the generating script's reference call and compares with the committed fixture (guards against a stale
-    fixture after an edit of the script)."""
+    """The outputs and gradients of each fixture are the reference module's, a fixed function of what the generating
+    script feeds it: the inputs, the loss weights and the Wigner-D matrices its e3nn stub hands over (computed by
+    pf3plat_b200.sh_rotation).  The fixture stays what the reference produces as long as the script still generates
+    the stored ones to fp32 rounding: guards against a stale fixture after an edit of the script or of sh_rotation."""
     sys.path.insert(0, au.GOLDEN)
-    saved = {k: v for k, v in sys.modules.items() if k == "src" or k.startswith("src.") or k.startswith("e3nn")}
-    try:
-        import make_adapter_golden as mk
-        ref = mk.load_reference_adapter()
-        seed, b, v, h, w, deg, proper = mk.CASES["adapter_pf3plat"]
+    import make_adapter_golden as mk
+    for name in au.CASES:
+        z, meta = au.load(name)
+        seed, b, v, h, w, deg, proper = mk.CASES[name]
+        assert (b, v, h, w, deg, proper) == tuple(meta.values()), name
         inp = mk.make_inputs(seed, b, v, h, w, deg, proper)
-        adapter = ref.GaussianAdapter(ref.GaussianAdapterCfg(gaussian_scale_min=0.5, gaussian_scale_max=15.0, sh_degree=deg))
-        out = adapter.forward(inp["extrinsics"], inp["intrinsics"], inp["coordinates"], inp["depths"], inp["opacities"],
-                              inp["raw_gaussians"], (h, w))
-        z, _ = au.load("adapter_pf3plat")
-        for k in au.OUTPUTS:
-            np.testing.assert_allclose(getattr(out, k).numpy(), z["out_" + k], rtol=1e-6, atol=1e-7)
-    finally:
-        for k in [k for k in sys.modules if k == "src" or k.startswith("src.") or k.startswith("e3nn")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+
+        def same(got, key):
+            np.testing.assert_allclose(got.numpy(), z[key], rtol=1e-6, atol=1e-7, err_msg=f"{name} {key}")
+        for k in au.INPUTS:
+            same(inp[k], "in_" + k)
+        for k, t in mk.make_weights(seed, {k: z["out_" + k].shape for k in au.OUTPUTS}).items():
+            same(t, "w_" + k)
+        same(mk.sh_rotation_used(inp["extrinsics"], b, v, deg), "sh_rotation")

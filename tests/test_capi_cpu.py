@@ -5,8 +5,8 @@ import ctypes
 import os
 import re
 import subprocess
-import sys
 
+import numpy as np
 import pytest
 import torch
 
@@ -118,46 +118,40 @@ def test_product_code_never_touches_the_oracle():
     assert not bad, bad
 
 
-REF = "/root/reference/src/model/decoder/cuda_splatting.py"
+OPERATOR_CALLS = os.path.join(ROOT, "tests", "golden", "operator_calls.npz")
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference tree only exists in the build container")
+def _recorded_operator_calls():
+    """(settings kwargs, call kwargs) of every operator call in tests/golden/operator_calls.npz, with the Python types
+    and requires_grad flags the reference passed."""
+    import json
+    z = np.load(OPERATOR_CALLS)
+    calls = {}
+    for key, kind in json.loads(str(z["kinds"])).items():
+        i, part, name = key.split(".")
+        if kind == "none":
+            v = None
+        elif kind.startswith("tensor"):
+            v = torch.from_numpy(z[key]).requires_grad_(kind == "tensor_grad")
+        else:
+            v = {"int": int, "float": float, "bool": bool}[kind](z[key])
+        calls.setdefault(int(i[1:]), ({}, {}))[part == "call"][name] = v
+    return [calls[i] for i in sorted(calls)]
+
+
 def test_reference_render_glue_imports_and_reaches_our_operator_unmodified():
-    """Imports the reference's cuda_splatting.py UNMODIFIED against this repo's `diff_gaussian_rasterization`
-    and drives render_cuda with CPU tensors: all of the reference's own glue runs and the call arrives at our
-    operator, which refuses CPU tensors loudly.  (The same call pattern is exercised on the GPU by
-    tests/test_gpu_dropin.py through a line-by-line restatement, since /root/reference is absent there.)"""
-    import importlib.util
-    import types
-    saved = {k: sys.modules.get(k) for k in list(sys.modules) if k == "src" or k.startswith("src.")}
-    try:
-        for name in ("src", "src.model", "src.model.decoder", "src.model.encoder", "src.model.encoder.costvolume",
-                     "src.geometry"):
-            m = types.ModuleType(name)
-            m.__path__ = [os.path.join("/root/reference", *name.split("."))]
-            sys.modules[name] = m
-        spec = importlib.util.spec_from_file_location("src.model.decoder.cuda_splatting", REF)
-        mod = importlib.util.module_from_spec(spec)
-        sys.modules[spec.name] = mod
-        spec.loader.exec_module(mod)
-        from pf3plat_b200.synthetic import make_scene
-        sc = make_scene(64, 2, 32, 32)
-        rep = lambda t: t[None].expand(2, *t.shape)
+    """Replays, with CPU tensors, the operator calls the reference's cuda_splatting.py made through the
+    `diff_gaussian_rasterization` names (tests/golden/operator_calls.npz, recorded by make_camera_golden.py from
+    render_cuda, render_depth_cuda and render_cuda_orthographic): the settings are built with the reference's
+    keywords and Python types, the rasterizer is called with its keywords, and every call arrives at our operator,
+    which refuses CPU tensors loudly.  (The same call pattern is exercised on the GPU by tests/test_gpu_dropin.py
+    through a line-by-line restatement of the reference's glue.)"""
+    import diff_gaussian_rasterization as dgr
+    calls = _recorded_operator_calls()
+    assert len(calls) == 5
+    # render_cuda_orthographic hands 0-dim tensors as tanfovx / tanfovy, the other call sites Python floats
+    assert isinstance(calls[-1][0]["tanfovx"], torch.Tensor) and isinstance(calls[0][0]["tanfovx"], float)
+    for settings, call in calls:
+        rasterizer = dgr.GaussianRasterizer(dgr.GaussianRasterizationSettings(**settings))
         with pytest.raises(RuntimeError, match="no CPU fallback"):
-            mod.render_cuda(sc.extrinsics, sc.intrinsics, sc.near, sc.far, sc.image_shape, sc.background,
-                            rep(sc.means), rep(sc.covariances), rep(sc.harmonics), rep(sc.opacities))
-        # the other two call sites of the extension (:192-217 with 0-dim tensor tanfov, :255-268 via render_depth_cuda)
-        with pytest.raises(RuntimeError, match="no CPU fallback"):
-            mod.render_depth_cuda(sc.extrinsics, sc.intrinsics, sc.near, sc.far, sc.image_shape, rep(sc.means),
-                                  rep(sc.covariances), rep(sc.opacities), mode="disparity")
-        one = lambda t: t[:1]
-        with pytest.raises(RuntimeError, match="no CPU fallback"):
-            mod.render_cuda_orthographic(one(sc.extrinsics), torch.tensor([2.0]), torch.tensor([2.0]), one(sc.near),
-                                         one(sc.far), sc.image_shape, one(sc.background), one(rep(sc.means)),
-                                         one(rep(sc.covariances)), one(rep(sc.harmonics)), one(rep(sc.opacities)))
-    finally:
-        for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-            del sys.modules[k]
-        for k, v in saved.items():
-            if v is not None:
-                sys.modules[k] = v
+            rasterizer(**call)
