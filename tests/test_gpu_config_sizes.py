@@ -14,66 +14,16 @@ import numpy as np
 import pytest
 import torch
 
-from pf3plat_b200.synthetic import make_pixel_aligned_scene, make_scene, make_target
-from tests.util import (SH_BANDS, affected_gaussians, check_grad, check_image_strict, oracle_view)
+from pf3plat_b200.synthetic import make_pixel_aligned_scene, make_scene
+from tests.util import check_image_strict, fwd_bwd_vs_oracle, gpu_device as _dev, oracle_view, render_scene as _render
 
 pytestmark = pytest.mark.gpu
-
-
-def _dev():
-    assert torch.cuda.is_available(), "GPU test needs CUDA"
-    return torch.device("cuda:0")
-
-
-def _render(sc, dev, with_depth=False, requires_grad=False):
-    from pf3plat_b200.render import render_views
-    d = sc.to(dev)
-    leaves = {"means": d.means[None].clone(), "cov": d.covariances[None].clone(), "sh": d.harmonics[None].clone(),
-              "opac": d.opacities[None].clone()}
-    if requires_grad:
-        for t in leaves.values():
-            t.requires_grad_(True)
-    out = render_views(d.extrinsics, d.intrinsics, d.near, d.far, d.image_shape, d.background, leaves["means"],
-                       leaves["cov"], leaves["sh"], leaves["opac"], with_depth=with_depth)
-    return out, leaves
-
-
-def _cov6(G):
-    G = G.detach().cpu().numpy()
-    return np.stack([G[:, 0, 0], G[:, 0, 1], G[:, 0, 2], G[:, 1, 1], G[:, 1, 2], G[:, 2, 2]], -1)
-
-
-def _fwd_bwd_vs_oracle(sc, views, max_fragile_frac, label):
-    dev = _dev()
-    h, w = sc.image_shape
-    color, leaves = _render(sc, dev, requires_grad=True)
-    target = make_target(views, h, w).to(dev)
-    ((color - target) ** 2).mean().backward()
-    P = sc.means.shape[0]
-    gm = np.zeros((P, 3)); go = np.zeros(P); gs = np.zeros((P, 25, 3)); gc = np.zeros((P, 6))
-    affected = np.zeros(P, bool)
-    for v in range(views):
-        orc = oracle_view(sc, v)
-        check_image_strict(color[v], orc, max_fragile_frac, f"{label} view {v}")
-        # gradients are compared on the oracle's own image (dL/dC from the oracle's colours), like the small tests
-        dL = (2 * (orc.color - target[v].cpu().numpy()) / target.numel()).astype(np.float32)
-        g = orc.backward(dL)
-        gm += g["means3D"]; go += g["opacities"][:, 0]; gs += g["shs"]; gc += g["cov3D_precomp"]
-        affected |= affected_gaussians(orc, orc.px_fragile) | orc.geom_fragile
-        orc.close()
-    print(f"[parity] {label}: {int(affected.sum())} of {P} Gaussians contribute to a fragile pixel")
-    check_grad(f"{label} dL/dmeans3D", leaves["means"].grad[0], gm, affected)
-    check_grad(f"{label} dL/dopacities", leaves["opac"].grad[0].reshape(P, 1), go.reshape(P, 1), affected)
-    gsh = leaves["sh"].grad[0].permute(0, 2, 1)          # (P, 25, 3)
-    check_grad(f"{label} dL/dshs", gsh, gs, affected, bands=SH_BANDS)
-    assert float(gsh[:, 16:].abs().max()) == 0.0 and np.abs(gs[:, 16:]).max() == 0.0   # bands the evaluator never reads
-    check_grad(f"{label} dL/dcov3D", _cov6(leaves["cov"].grad[0]), gc, affected)
 
 
 def test_c3_forward_and_all_gradients_at_config_size():
     """BASELINE.json configs[2]: 500k Gaussians, 256x256, forward+backward (MSE to a random target); 2 of the 8 views."""
     sc = make_scene(500_000, 2, 256, 256, seed=0, total_views=8)
-    _fwd_bwd_vs_oracle(sc, 2, max_fragile_frac=0.03, label="C3")
+    fwd_bwd_vs_oracle(sc, 2, max_fragile_frac=0.03, label="C3")
 
 
 def test_c5_shape_forward_and_gradients():
@@ -81,7 +31,7 @@ def test_c5_shape_forward_and_gradients():
     sc = make_pixel_aligned_scene(256, 256, 2, seed=5)
     assert sc.means.shape[0] == 2 * 256 * 256
     # sub-pixel splats on a smooth surface put more pixels next to an alpha = 1/255 contour: 3.3 % fragile (C3: 1.2 %)
-    _fwd_bwd_vs_oracle(sc, 2, max_fragile_frac=0.05, label="C5-shape")
+    fwd_bwd_vs_oracle(sc, 2, max_fragile_frac=0.05, label="C5-shape")
 
 
 def test_c4_forward_and_depth_at_config_size():

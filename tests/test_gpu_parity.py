@@ -293,8 +293,10 @@ def test_compositor_variants_agree():
     from pf3plat_b200.cameras import make_view_batch
     from pf3plat_b200.rasterizer import BatchSettings, rasterize_batch
     dev = _dev()
+    from tests.util import make_posed_scene
     for sc, depth in ((make_scene(40000, 3, 80, 112, seed=12), True), (make_scene(300, 1, 16, 16, seed=13), False),
-                      (make_scene(150000, 2, 128, 128, seed=14), False)):
+                      (make_scene(150000, 2, 128, 128, seed=14), False),
+                      (make_posed_scene(40000, 4, 80, 112, seed=12), True)):   # rotated views, near != 1, clamped
         d = sc.to(dev)
         vb = make_view_batch(d.extrinsics, d.intrinsics, d.near, d.far)
         h, w = sc.image_shape

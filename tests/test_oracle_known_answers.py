@@ -191,3 +191,143 @@ def test_tile_lists_are_in_depth_then_index_order_for_any_thread_count():
         gs_oracle.set_threads(prev)
     for pl, rg, col in lists[1:]:
         assert np.array_equal(pl, lists[0][0]) and np.array_equal(rg, lists[0][1]) and np.array_equal(col, lists[0][2])
+
+
+# ---------------------------------------------------------------------------------------------------------
+# rotated cameras: pose convention, rotation equivariance, the roles of x and y, the guard band
+# ---------------------------------------------------------------------------------------------------------
+def _one_view_scene(c2w, fx, fy, h, w, means, cov, colors, opac, near=1.0, bg=(0.2, 0.3, 0.4)):
+    """A one-view fp64 Scene (colours as degree-0 'harmonics', read back by view_args(use_sh=False))."""
+    import torch
+
+    from pf3plat_b200.synthetic import Scene
+    t = lambda a: torch.as_tensor(np.asarray(a), dtype=torch.float64)
+    K = np.array([[fx, 0, 0.5], [0, fy, 0.5], [0, 0, 1.0]])
+    P = len(means)
+    return Scene(t(c2w)[None], t(K)[None], t([near]), t([100.0]), (h, w), t(bg)[None], t(means), t(cov),
+                 t(colors)[:, :, None], t(opac), torch.zeros(P, 3, dtype=torch.float64), torch.zeros(P, 4, dtype=torch.float64))
+
+
+def _render(sc, dt=np.float64, **extra):
+    from tests.util import view_args
+    st, kw = view_args(sc, 0, use_sh=False)
+    return OracleRender(st, dtype=dt, **kw, **extra), st
+
+
+@pytest.mark.parametrize("dt", DT)
+def test_pose_convention_end_to_end(dt):
+    """c2w = yaw 90 + pitch 30 at c != 0, through make_view_batch (itself pinned to the reference's glue by
+    camera_glue.npz): a Gaussian at c + d * forward lands on the image centre, + delta * right moves it right by
+    fx_px * delta / d pixels, + delta * down moves it down by fy_px * delta / d."""
+    from tests.util import posed_c2w
+    c2w = posed_c2w(90.0, 30.0, 0.0)
+    c = np.array([1.5, -0.7, 2.0])
+    c2w[:3, 3] = c
+    h, w, fx, fy = 64, 80, 0.8, 1.1
+    d, delta = 6.0, 0.25
+    R = c2w[:3, :3]
+    means = np.stack([c + d * R[:, 2], c + d * R[:, 2] + delta * R[:, 0], c + d * R[:, 2] + delta * R[:, 1]])
+    cov = np.repeat((0.02 ** 2 * np.eye(3))[None], 3, 0)
+    r, _ = _render(_one_view_scene(c2w, fx, fy, h, w, means, cov, np.ones((3, 3)), np.full(3, 0.5)), dt)
+    centre = np.array([(w - 1) / 2, (h - 1) / 2])
+    assert (r.radii > 0).all()
+    assert np.allclose(r.xy[0], centre, atol=1e-4)
+    assert np.allclose(r.xy[1], centre + [fx * w * delta / d, 0], atol=1e-4)
+    assert np.allclose(r.xy[2], centre + [0, fy * h * delta / d], atol=1e-4)
+    assert np.allclose(r.depths, d, rtol=1e-6)
+
+
+def _random_rotation(rng):
+    q, _ = np.linalg.qr(rng.standard_normal((3, 3)))
+    return q * np.sign(np.linalg.det(q))
+
+
+def test_rotation_equivariance():
+    """The same world rotation applied to the means, the covariances and the camera leaves the fp64 image (outside
+    fragile pixels) and the radii unchanged -- for every view of a posed scene, Gaussians behind the camera, in the
+    near cull and past the guard band included.  A view block read transposed anywhere breaks this."""
+    import torch
+
+    from pf3plat_b200.synthetic import Scene
+    from tests.util import make_posed_scene, view_args
+    sc = make_posed_scene(3000, 4, 64, 80, seed=21)
+    sc = Scene(**{k: (v.double() if torch.is_tensor(v) else v) for k, v in sc.__dict__.items()})
+    Q = torch.tensor(_random_rotation(np.random.default_rng(4)))
+    ext = sc.extrinsics.clone()
+    ext[:, :3, :3] = Q @ ext[:, :3, :3]
+    ext[:, :3, 3] = ext[:, :3, 3] @ Q.T
+    rot = Scene(**{**sc.__dict__, "extrinsics": ext, "means": sc.means @ Q.T, "covariances": Q @ sc.covariances @ Q.T})
+    for v in range(4):
+        a = OracleRender(*_args(view_args(sc, v, use_sh=False)), dtype=np.float64)
+        b = OracleRender(*_args(view_args(rot, v, use_sh=False)), dtype=np.float64)
+        frag = a.px_fragile | b.px_fragile
+        assert frag.mean() < 0.05 and a.num_rendered > 1000
+        assert np.abs(a.color - b.color).max(axis=0)[~frag].max() < 1e-9
+        assert np.array_equal(a.radii, b.radii)
+
+
+def _args(st_kw):
+    st, kw = st_kw
+    return (st,) + tuple(kw[k] for k in ("means3D", "opacities")) + (None, kw["colors_precomp"], None, None, kw["cov3D_precomp"])
+
+
+@pytest.mark.parametrize("dt", DT)
+def test_roll_by_90_degrees_rotates_the_image(dt):
+    """Rolling the camera by 90 degrees about its axis, with H <-> W and fx <-> fy swapped, gives np.rot90 of the image:
+    fixes which of tanfovx / tanfovy, limx / limy and W / H goes with which image axis.  Footprints are >= 5 px and
+    opacities < 0.19, so no Gaussian reaches alpha 1/255 where the tile rectangle (not mirror-symmetric) cuts it off;
+    widths are multiples of 16, so the tile grids map onto each other; some Gaussians sit past the guard band."""
+    from tests.util import posed_c2w
+    rng = np.random.default_rng(8)
+    h, w, fx, fy = 64, 96, 0.7, 1.2            # tanfovx = 0.71, tanfovy = 0.42
+    tx, ty = 0.5 / fx, 0.5 / fy
+    n = 120
+    z = rng.uniform(3, 9, n)
+    rx = np.where(np.arange(n) % 6 == 0, rng.choice([-1, 1], n) * rng.uniform(1.4, 1.9, n), rng.uniform(-1, 1, n))
+    ry = np.where(np.arange(n) % 6 == 1, rng.choice([-1, 1], n) * rng.uniform(1.4, 1.9, n), rng.uniform(-1, 1, n))
+    cam = np.stack([rx * tx * z, ry * ty * z, z], -1)
+    sig = rng.uniform(5, 12, n) * z / (fx * w) * np.where(np.abs(rx) > 1.3, 4, 1)
+    A = rng.standard_normal((n, 3, 3)) * 0.3 + np.eye(3)
+    cov = np.einsum("nij,nkj->nik", A, A) * (sig ** 2)[:, None, None]
+    cols, opac = rng.uniform(0, 1, (n, 3)), rng.uniform(0.03, 0.19, n)
+    c2w = posed_c2w(25.0, -15.0, 10.0)
+    means = c2w[:3, 3] + cam @ c2w[:3, :3].T
+    a, sa = _render(_one_view_scene(c2w, fx, fy, h, w, means, cov, cols, opac), dt)
+    c2w_b = c2w.copy()
+    c2w_b[:3, :3] = c2w[:3, :3] @ np.array([[0.0, -1, 0], [1, 0, 0], [0, 0, 1]])
+    b, sb = _render(_one_view_scene(c2w_b, fy, fx, w, h, means, cov, cols, opac), dt)
+    assert abs(sb.tanfovx - sa.tanfovy) < 1e-12 and abs(sb.tanfovy - sa.tanfovx) < 1e-12 and sa.tanfovx != sa.tanfovy
+    rot = np.rot90(a.color, 1, axes=(1, 2))
+    frag = np.rot90(a.px_fragile) | b.px_fragile
+    assert b.color.shape == rot.shape and frag.mean() < 0.05
+    assert np.abs(b.color - rot).max(axis=0)[~frag].max() < (1e-9 if dt == np.float64 else 2e-5)
+    assert np.array_equal(a.radii, b.radii) and (a.radii > 0).sum() > 0.9 * n
+
+
+@pytest.mark.parametrize("dt", DT)
+def test_guard_band_clamp(dt):
+    """A Gaussian at x/z = 2 limx (limx = 1.3 tanfovx): its 2D covariance is J Sigma J^T + 0.3 I with J taken at the
+    CLAMPED position (t.x = limx t.z); in the backward, nothing reaches mean.x through J (the clamped axis), only through
+    means2D -- while mean.y, inside the band, gets both."""
+    tanfov, z = 0.5, 4.0
+    st = simple_settings(48, 64, tanfov=tanfov, bg=(0.1, 0.2, 0.3))
+    limx = 1.3 * tanfov
+    mean = np.array([2 * limx * z, 0.3 * tanfov * z, z])
+    L = np.array([[0.9, 0, 0], [0.4, 0.6, 0], [-0.3, 0.5, 0.7]])
+    Sigma = L @ L.T * 1.5
+    c6 = Sigma[np.triu_indices(3)][None]
+    r = OracleRender(st, means3D=mean[None], opacities=np.array([0.8]), colors_precomp=np.array([[0.9, 0.4, 0.1]]),
+                     cov3D_precomp=c6, dtype=dt)
+    assert r.radii[0] > 0
+    fx, fy = 64 / (2 * tanfov), 48 / (2 * tanfov)
+    J = np.array([[fx / z, 0, -fx * limx * z / z ** 2], [0, fy / z, -fy * mean[1] / z ** 2]])
+    cov2 = J @ Sigma @ J.T + 0.3 * np.eye(2)
+    inv = np.linalg.inv(cov2)
+    assert np.allclose(r.conic_opacity[0, :3], [inv[0, 0], inv[0, 1], inv[1, 1]], rtol=1e-5)
+    g = r.backward(np.random.default_rng(0).standard_normal((3, 48, 64)))
+    # identity view: dL/dmean.x = (through J: masked) + d ndc_x / d mean.x * dL/dmeans2D.x = (1 / tanfov) / z * ...
+    gx_proj = (1 / tanfov) / z * g["means2D"][0, 0]
+    gy_proj = (1 / tanfov) / z * g["means2D"][0, 1]
+    assert abs(g["means2D"][0, 0]) > 1e-3
+    assert np.isclose(g["means3D"][0, 0], gx_proj, rtol=1e-5, atol=1e-9)
+    assert abs(g["means3D"][0, 1] - gy_proj) > 1e-2 * abs(g["means3D"][0, 1])
